@@ -30,6 +30,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the tree may be read-only: bench.py writes nothing into it
 
 METRIC = "visits/sec 19x19 b18c384nbt selfplay"
 UNIT = "visits/s"
@@ -58,7 +59,12 @@ def parse_args():
     ap.add_argument("--mixed-sizes", action="store_true", help="BASELINE.json configs[3]: every game draws its board from 9x9 / 13x13 / 19x19 (equal "
                     "probabilities, like bSizes = 9,13,19) inside the 19x19 evaluator frame; a finished game's slot draws again")
     ap.add_argument("--visits", type=int, default=600, help="maxVisits per move (BASELINE.json configs[1]: 600)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the device loop's last wave left for its caller (roots, boards, leaf rows) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def load_peaks():
@@ -264,6 +270,37 @@ def _nbytes(x):
     return 8 if isinstance(x, (int, float, bool)) else 0
 
 
+DUMP_MAX_GAMES = 256
+
+
+def dump_outputs(sp, out_dir, world):
+    """What a caller of the device loop reads back after its last wave: per game the root's children (visits, prior policy, utility),
+    their value statistics, the root's own, the board and game state, and the NN row the wave evaluated; plus the loop's counters.
+    Integer and float32 arrays are written as float32 (exact: every count stays below 2^24), the loop's doubles as float64.  More than
+    DUMP_MAX_GAMES games over all ranks: a fixed sample of each rank's games (seed 0), listed in games.npy, keeps the files of all
+    ranks together near 14 MB."""
+    n, keep = sp.num_games, max(1, DUMP_MAX_GAMES // world)
+    games = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    cols = {k: [] for k in ("child_visits", "child_policy", "child_utility", "child_value_stats", "root_value_stats", "board", "game_info",
+                            "nn_row_spatial", "nn_row_global")}
+    for g in games:
+        visits, policy, util = sp.root_children(int(g))
+        ch, rt = sp.root_value_stats(int(g))
+        colors, info = sp.game(int(g))
+        spatial, glob = sp.nn_row(int(g))
+        for k, v in (("child_visits", visits), ("child_policy", policy), ("child_utility", util), ("child_value_stats", ch), ("root_value_stats", rt),
+                     ("board", colors), ("game_info", list(info.values())), ("nn_row_spatial", spatial), ("nn_row_global", glob)):
+            cols[k].append(v)
+    out = {k: np.asarray(v, np.float64 if k in ("child_utility", "child_value_stats", "root_value_stats") else np.float32) for k, v in cols.items()}
+    out["games"] = games.astype(np.float32)
+    out["root_visits"] = sp.root_visits()[games].astype(np.float32)
+    out["nn_symmetries"] = sp.nn_symmetries()[games].astype(np.float32)
+    out["stats"] = np.array(list(sp.stats().values()), np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v)
+
+
 def main():
     args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
@@ -347,7 +384,7 @@ def main():
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
-    W, K = max(3, args.warmup), max(1, args.steps)
+    W, K = max(3, args.warmup), args.steps
     # device-resident self-play loop: selfplay8mainb18.cfg search parameters that the loop implements (DESIGN.md §8)
     sp_kwargs = dict(komi=7.5, multi_stone_suicide_legal=True, early_temperature_moves=30,
                   cpuct_exploration=1.05, cpuct_exploration_log=0.28, cpuct_exploration_base=500.0, fpu_reduction_max=0.2,
@@ -388,6 +425,8 @@ def main():
     ms_dev = timed(lambda i: sp.run(1), K)
     clocks = sampler.stop() if rank == 0 else None
     after = sp.stats()
+    if args.dump_outputs:
+        dump_outputs(sp, os.path.join(args.dump_outputs, f"rank{rank}") if world > 1 else args.dump_outputs, world)
     # a wave delivers one evaluated leaf per game, except for games whose ladder searches are still running (stalled_waves);
     # under graph search a game can also finish extra playouts inside the wave on edges that only need to catch up
     done = after["total_visits"] - before["total_visits"]
@@ -439,9 +478,8 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record(stream)
-    pumps = max(1, (K + PUMP - 1) // PUMP)
-    for _ in range(pumps):
-        rec.pump(PUMP)
+    for first in range(0, K, PUMP):
+        rec.pump(min(PUMP, K - first))
     e1.record(stream)
     handle.sync()
     barrier()
@@ -455,7 +493,6 @@ def main():
     if world > 1:
         dist.all_reduce(rec_visits, op=dist.ReduceOp.SUM)
     rec_visits = float(rec_visits.item())
-    rec_waves = pumps * PUMP + 0          # + the extra waves in which released games moved (counted from the stats below)
     rec_moves, rec_games, rec_rows = rec.moves_recorded - moves0, rec.games_written - games0, writer.row_count - rows0
     writer.flush_if_nonempty()
     rec_files = len([f for f in os.listdir(out_dir) if f.endswith(".npz")])
@@ -519,7 +556,9 @@ def main():
         achieved = conv_flop / (float(ms_conv[0]) * 1e-3) / 1e12
         whole = flop_per_eval * n * K / (ms_nn * 1e-3) / 1e12
         cpu_obj = {"value": None, "unit": UNIT, "cores": 0, "kind": "reference", "sample": "measured at N=1 only"}
-        if world == 1:      # the CPU baseline is a property of the box: measured at N=1 only
+        if world == 1 and not os.path.exists(CPU_SELFPLAY):       # the CPU arm links the reference's sources: built only where they are present
+            cpu_obj["sample"] = "not measured: oracle/_ref/kgref_cpu_selfplay is not built"
+        elif world == 1:      # the CPU baseline is a property of the box: measured at N=1 only
             cpu_obj = cpu_baseline_object(cpu_selfplay(args.model, 15.0, 5.0, args.visits), args.model)
         out = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
@@ -551,8 +590,8 @@ def main():
                                   "game_waves": n * K},
                        "weight_broadcast_ms": bcast_ms, "weight_broadcast": bcast, "gpu_competitor": competitor},
             "value_fp32_equivalent": value_fp32,
-            "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": slots.h2d / (pumps * PUMP), "d2h_bytes_per_step": slots.d2h / (pumps * PUMP),
-                    "ms_per_step": ms_rec / (pumps * PUMP),
+            "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": slots.h2d / K, "d2h_bytes_per_step": slots.d2h / K,
+                    "ms_per_step": ms_rec / K,
                     "what": "device loop in hold mode + GameRecorder.pump (per-game release every 8 waves: root readback, training targets) + TrainingDataWriter "
                             ".npz files; host work inside the timed region; a step = one playout wave (the wave in which released games move is extra)",
                     "moves_recorded": rec_moves, "games_finished": rec_games, "rows_written": rec_rows, "npz_files": rec_files, "frac_of_value": e2e_value / value,

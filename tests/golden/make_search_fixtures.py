@@ -37,7 +37,8 @@ LCB = {"useLcbForSelection": 1, "lcbStdevs": 5.0, "minVisitPropForLCB": 0.15, "u
 BIAS = {"subtreeValueBiasFactor": 0.30, "subtreeValueBiasWeightExponent": 0.8}
 
 
-def run(X, Y, visits, moves, score=None, driver=None, model=None, env=None, frame=None):
+def run(X, Y, visits, moves, score=None, driver=None, model=None, env=None, frame=None, answer=None):
+    """answer(args, env) -> the driver's stdout, in place of running it (tests: the stored answers of tests/reference_runs.py)."""
     s = " ".join("pass" if m is None else f"{m[0]},{m[1]}" for m in moves)
     if score is None:
         score = {}
@@ -46,8 +47,11 @@ def run(X, Y, visits, moves, score=None, driver=None, model=None, env=None, fram
     extra = [f"{k}={float(v)!r}" for k, v in score.items() if k != "fullHistoryRules"]
     if frame is not None:      # the evaluator's frame is frame x frame, the board X x Y in its corner: positions are y * frame + x
         env = dict(env or {}, KGREF_NN_LEN=str(frame))
-    out = subprocess.run([driver or DRIVER, "searchfake", model or MODEL, str(X), str(Y), str(visits), s] + extra, capture_output=True, text=True, check=True,
-                         env=(dict(os.environ, **env) if env else None)).stdout
+    args = ["searchfake", model or MODEL, str(X), str(Y), str(visits), s] + extra
+    if answer is not None:
+        out = answer(args, env)
+    else:
+        out = subprocess.run([driver or DRIVER] + args, capture_output=True, text=True, check=True, env=(dict(os.environ, **env) if env else None)).stdout
     bx = X
     if frame is not None:
         X = Y = frame

@@ -13,20 +13,23 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-REF = "/root/reference/cpp"
+MOCK = os.path.join(ROOT, "oracle", "_ref", "kgb200_mock.o")
 REF_LIB = os.path.join(ROOT, "oracle", "_ref", "libkgref.a")
 
-pytestmark = pytest.mark.skipif(not (os.path.isdir(REF) and os.path.exists(REF_LIB)), reason="needs the reference sources and oracle/_ref/libkgref.a (the mock plays on the reference's Board)")
+pytestmark = pytest.mark.skipif(not (os.path.exists(MOCK) and os.path.exists(REF_LIB)),
+                                reason="oracle/_ref/kgb200_mock.o is not built (oracle/Makefile.drivers compiles the mock against the reference's sources)")
+
+
+def _host_on_mock(main_src, exe):
+    """A C++ host - repository sources only - linked against the mock of the recording ABI and the reference objects the mock plays on."""
+    subprocess.run(["g++", "-O1", "-std=c++17", "-mfpmath=sse", "-DNDEBUG", "-w", "-I" + ROOT, "-o", str(exe), os.path.join(ROOT, "integration", main_src), MOCK,
+                    "-Wl,--start-group", REF_LIB, "-Wl,--end-group", "-lz", "-lpthread"], check=True, cwd=ROOT)
+    return str(exe)
 
 
 @pytest.fixture(scope="module")
 def host_on_mock(tmp_path_factory):
-    exe = tmp_path_factory.mktemp("cpphost_mock") / "b200_selfplay_mock"
-    subprocess.run(["g++", "-O1", "-std=c++17", "-mfpmath=sse", "-DNDEBUG", "-DNO_GIT_REVISION", "-DNO_LIBZIP", "-w", "-I" + REF, "-I" + REF + "/external",
-                    "-isystem", REF + "/external/tclap-1.2.5/include", "-isystem", REF + "/external/filesystem-1.5.8/include", "-I" + ROOT, "-o", str(exe),
-                    os.path.join(ROOT, "integration", "b200_selfplay_main.cpp"), os.path.join(ROOT, "tests", "mock", "kgb200_mock.cpp"),
-                    "-Wl,--start-group", REF_LIB, "-Wl,--end-group", "-lz", "-lpthread"], check=True, cwd=ROOT)
-    return str(exe)
+    return _host_on_mock("b200_selfplay_main.cpp", tmp_path_factory.mktemp("cpphost_mock") / "b200_selfplay_mock")
 
 
 def _replay_slots_with_limits(log, G, size, V, uneven=0):
@@ -420,12 +423,7 @@ def test_cpp_host_ranks_swap_nets_together_under_nccl_weights(tmp_path, host_on_
 
 @pytest.fixture(scope="module")
 def gatekeeper_on_mock(tmp_path_factory):
-    exe = tmp_path_factory.mktemp("cppgate_mock") / "b200_gatekeeper_mock"
-    subprocess.run(["g++", "-O1", "-std=c++17", "-mfpmath=sse", "-DNDEBUG", "-DNO_GIT_REVISION", "-DNO_LIBZIP", "-w", "-I" + REF, "-I" + REF + "/external",
-                    "-isystem", REF + "/external/tclap-1.2.5/include", "-isystem", REF + "/external/filesystem-1.5.8/include", "-I" + ROOT, "-o", str(exe),
-                    os.path.join(ROOT, "integration", "b200_gatekeeper_main.cpp"), os.path.join(ROOT, "tests", "mock", "kgb200_mock.cpp"),
-                    "-Wl,--start-group", REF_LIB, "-Wl,--end-group", "-lz", "-lpthread"], check=True, cwd=ROOT)
-    return str(exe)
+    return _host_on_mock("b200_gatekeeper_main.cpp", tmp_path_factory.mktemp("cppgate_mock") / "b200_gatekeeper_mock")
 
 
 @pytest.mark.parametrize("uneven", [0, 9], ids=["instant_searches", "uneven_searches"])
@@ -487,11 +485,7 @@ def test_cpp_match_plays_two_named_bots_like_the_python_match(tmp_path, uneven):
     """`katago match` for two named bots as a C++-only host (integration/b200_match_main.cpp): per-bot search keys (maxVisits0 / maxVisits1), alternating
     colours, per-game setups - against the Python match engine on the mock loops' logs: the record file character for character, the same wins and points."""
     import re
-    exe = tmp_path / "b200_match_mock"
-    subprocess.run(["g++", "-O1", "-std=c++17", "-mfpmath=sse", "-DNDEBUG", "-DNO_GIT_REVISION", "-DNO_LIBZIP", "-w", "-I" + REF, "-I" + REF + "/external",
-                    "-isystem", REF + "/external/tclap-1.2.5/include", "-isystem", REF + "/external/filesystem-1.5.8/include", "-I" + ROOT, "-o", str(exe),
-                    os.path.join(ROOT, "integration", "b200_match_main.cpp"), os.path.join(ROOT, "tests", "mock", "kgb200_mock.cpp"),
-                    "-Wl,--start-group", REF_LIB, "-Wl,--end-group", "-lz", "-lpthread"], check=True, cwd=ROOT)
+    exe = _host_on_mock("b200_match_main.cpp", tmp_path / "b200_match_mock")
     from katago_b200 import match_cli as MC, selfplay_cli as C
     from katago_b200.game_initializer import GameInitializer
     from katago_b200.match_play import MatchPlay

@@ -4,7 +4,8 @@
   (itself pinned to the reference's tiny-net known answers and PyTorch model outputs, tests/test_oracle_nn.py) through the unmodified
   reference's NNResultBuf / NNOutput plumbing (oracle/ref_nnloop_driver.cpp), symmetries included;
 * the self-play driver: reference Search + Board + NNEvaluator on that backend completes visits and reports them.
-Needs the binaries under oracle/_ref/ (built where /root/reference exists; they travel with the snapshot)."""
+Both need the binaries under oracle/_ref/, built only where the reference's sources are; the backend's dumps are stored
+(tests/reference_runs.py), so the first test also runs without them."""
 import json
 import os
 import subprocess
@@ -17,20 +18,17 @@ import kg_nn_oracle as orc
 from katago_b200 import modelgen
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-NNLOOP = os.path.join(ROOT, "oracle", "_ref", "kgref_nnloop_cpu")
 SELFPLAY = os.path.join(ROOT, "oracle", "_ref", "kgref_cpu_selfplay")
 sys.path.insert(0, os.path.join(ROOT, "tests", "gpu_checks"))
-
-pytestmark = pytest.mark.skipif(not (os.path.exists(NNLOOP) and os.path.exists(SELFPLAY)), reason="oracle/_ref CPU baseline binaries are not built")
 
 
 @pytest.mark.parametrize("cfg", ["tiny_reg", "tiny_nbt", "mid_nbt"])
 def test_cpu_backend_matches_the_numpy_oracle(tmp_path, cfg):
     from competitor_parity import read
+    from reference_runs import reference_run
     path = modelgen.write_model(str(tmp_path / f"{cfg}.bin"), cfg, seed=4)
     dump = str(tmp_path / "dump.bin")
-    out = subprocess.run([NNLOOP, path, "6", "1", "0", "1", "1", dump], capture_output=True, text=True, timeout=300, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-    assert out.returncode == 0, out.stderr[-500:]
+    reference_run("kgref_nnloop_cpu", [path, 6, 1, 0, 1, 1, dump], env={"CUDA_VISIBLE_DEVICES": ""}, timeout=300)
     rows = read(dump)
     C = len(rows[0]["spatial"]) // 361
     sp = np.stack([r["spatial"].reshape(19, 19, C) for r in rows])
@@ -44,6 +42,7 @@ def test_cpu_backend_matches_the_numpy_oracle(tmp_path, cfg):
     assert np.abs(ref["ownership"].reshape(len(rows), -1) - np.stack([r["own"] for r in rows])).max() < 1e-4
 
 
+@pytest.mark.skipif(not os.path.exists(SELFPLAY), reason="oracle/_ref/kgref_cpu_selfplay is not built (it links the reference's sources)")
 def test_cpu_selfplay_driver_counts_visits(tmp_path):
     path = modelgen.write_model(str(tmp_path / "tiny.bin"), "tiny_reg", seed=3)
     out = subprocess.run([SELFPLAY, path, "3", "4", "2", "40", "9", "1", "20"], capture_output=True, text=True, timeout=300, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))

@@ -517,25 +517,17 @@ class ReplaySlots:
                     final_colors=np.array(m["final_colors"] or [0] * n, np.uint8), final_area=np.array(m["final_area"] or [0] * n, np.uint8))
 
 
-REF_LIB = os.path.join(ROOT, "oracle", "_ref", "libkgref.a")
-
-
-@pytest.mark.skipif(not (os.path.isdir("/root/reference/cpp") and os.path.exists(REF_LIB)), reason="needs the reference sources and oracle/_ref/libkgref.a")
 @pytest.mark.parametrize("size,ko_rule,komi,max_moves", [(9, 0, 6.5, 40), (5, 1, 7.0, 60)])
 def test_cpp_recorder_against_python_recorder_on_scripted_slots(tmp_path, size, ko_rule, komi, max_moves):
     """No GPU: oracle/ref_record_driver.cpp (integration/b200record.h + the reference's own TrainingDataWriter) linked against a CPU mock
-    of the recording ABI that plays random legal games on the reference's Board.  The C++ recorder's own checks (legality, game end,
-    final score and area) run on every move; its rows - planes recomputed by the reference - must equal the rows the Python recorder
-    and writer produce from the mock's log: input planes bit for bit, integer targets exactly, floats to the text sink's 6 digits."""
-    import ctypes, subprocess
+    of the recording ABI that plays random legal games on the reference's Board (oracle/_ref/kgref_record_mock; tests/reference_runs.py).
+    The C++ recorder's own checks (legality, game end, final score and area) ran on every move; its rows - planes recomputed by the
+    reference - must equal the rows the Python recorder and writer produce from the mock's log: input planes bit for bit, integer
+    targets exactly, floats to the text sink's 6 digits."""
+    import ctypes
     from katago_b200.nn_backend import SelfplayConfig
+    from reference_runs import reference_run
     from test_npz_writer import _parse_text_dump
-    ref = "/root/reference/cpp"
-    exe = tmp_path / "record_mock"
-    subprocess.run(["g++", "-O1", "-std=c++17", "-mfpmath=sse", "-DNDEBUG", "-DNO_GIT_REVISION", "-DNO_LIBZIP", "-w", "-I" + ref, "-I" + ref + "/external",
-                    "-isystem", ref + "/external/tclap-1.2.5/include", "-isystem", ref + "/external/filesystem-1.5.8/include", "-I" + ROOT, "-o", str(exe),
-                    os.path.join(ROOT, "oracle", "ref_record_driver.cpp"), os.path.join(ROOT, "tests", "mock", "kgb200_mock.cpp"),
-                    "-Wl,--start-group", REF_LIB, "-Wl,--end-group", "-lz", "-lpthread"], check=True, cwd=ROOT)
     G, V, NUM = 3, 20, 5
     c = SelfplayConfig()
     c.num_games, c.max_visits, c.max_moves, c.multi_stone_suicide_legal, c.komi, c.seed = G, V, max_moves, 1, komi, 5 + size
@@ -543,9 +535,7 @@ def test_cpp_recorder_against_python_recorder_on_scripted_slots(tmp_path, size, 
     (tmp_path / "cfg.bin").write_bytes(ctypes.string_at(ctypes.addressof(c), ctypes.sizeof(c)))
     (tmp_path / "model.bin").write_bytes(b"unused")
     log = tmp_path / "log.jsonl"
-    r = subprocess.run([str(exe), str(tmp_path / "model.bin"), str(size), str(tmp_path / "cfg.bin"), str(NUM), str(tmp_path / "rows.txt")],
-                       env=dict(os.environ, KGB_MOCK_LOG=str(log)), capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stderr[-2000:]
+    reference_run("kgref_record_mock", [tmp_path / "model.bin", size, tmp_path / "cfg.bin", NUM, tmp_path / "rows.txt"], env={"KGB_MOCK_LOG": log})
     want = _parse_text_dump((tmp_path / "rows.txt").read_text())
     assert len(want) == 1
 
@@ -578,10 +568,6 @@ def test_cpp_recorder_against_python_recorder_on_scripted_slots(tmp_path, size, 
     assert any(d.end_finished for d in games[:NUM]) or size == 9        # the small board also sees games that end by passes
 
 
-DRIVER = os.path.join(ROOT, "oracle", "_ref", "kgref_driver")
-
-
-@pytest.mark.skipif(not os.path.exists(DRIVER), reason="oracle/_ref/kgref_driver not built")
 @pytest.mark.parametrize("size,visits,max_moves,seed,psw,vsw", [(9, 40, 50, 3, 0.5, 0.1), (7, 60, 200, 12, 0.3, 0.2), (13, 25, 70, 5, 0.0, 0.0)])
 def test_recorder_chain_against_a_whole_reference_selfplay_game(tmp_path, size, visits, max_moves, seed, psw, vsw):
     """The whole host chain against the reference's own self-play: `kgref_driver rungame` plays a game with Play::runGame (CPU, fake
@@ -590,12 +576,11 @@ def test_recorder_chain_against_a_whole_reference_selfplay_game(tmp_path, size, 
     targets, game-end targets, surprise weights (left fractional on both sides, so the writers' identically seeded Rands decide the
     extra rows) and every addRow column.  Two documented differences: the Q targets are listed in position order here and in child
     creation order there, so their stochastic rounding may differ by one unit; and the three "raw net statistics" columns come from a
-    separate evaluation in the reference."""
-    import subprocess
+    separate evaluation in the reference.  The driver's log and rows are stored (tests/reference_runs.py)."""
+    from reference_runs import reference_run
     from test_npz_writer import _parse_text_dump
     log, rows = tmp_path / "slot.log", tmp_path / "rows.txt"
-    subprocess.run([DRIVER, "rungame", os.path.join(GOLDEN, "models", "torchref_b2c16.bin.gz"), str(size), str(visits), str(max_moves), str(seed),
-                    str(psw), str(vsw), "0", str(log), str(rows)], check=True, capture_output=True, timeout=300)
+    reference_run("kgref_driver", ["rungame", os.path.join(GOLDEN, "models", "torchref_b2c16.bin.gz"), size, visits, max_moves, seed, psw, vsw, 0, log, rows])
     want = _parse_text_dump(rows.read_text())
     assert len(want) == 1
     sp = ReplaySlots(str(log), 1, size, visits)
@@ -743,13 +728,11 @@ def test_recorded_games_through_the_reference_writer(tmp_path, tmp_models, ko_ru
     recomputed by the reference's fillRowV7 on its own Board / BoardHistory, every move re-checked by its isLegal, game end and
     final score by its BoardHistory.  The same configuration recorded by katago_b200/game_recorder.py + npz_writer.py must give the
     same rows: input planes bit for bit (the device's featurization of whole games vs the reference's), integer targets exactly,
-    float columns to the 6 digits of the reference's text sink."""
-    import ctypes, subprocess
+    float columns to the 6 digits of the reference's text sink.  The reference's rows are stored (tests/reference_runs.py)."""
+    import ctypes
     from katago_b200.nn_backend import NeuralNet, SelfPlay
+    from reference_runs import reference_run
     from test_npz_writer import _parse_text_dump
-    exe = os.path.join(ROOT, "oracle", "_ref", "kgref_record")
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/kgref_record not built (needs the reference sources at build time)")
     L, G, V, NUM = 9, 6, 40, 6
     komi = 7.0 if ko_rule else 6.5
     lm = NeuralNet.loadModelFile(tmp_models["tiny_reg"])
@@ -764,8 +747,7 @@ def test_recorded_games_through_the_reference_writer(tmp_path, tmp_models, ko_ru
     cfg_path = tmp_path / "config.bin"
     cfg_path.write_bytes(ctypes.string_at(ctypes.addressof(sp.cfg), ctypes.sizeof(sp.cfg)))
     out_path = tmp_path / "reference_rows.txt"
-    r = subprocess.run([exe, tmp_models["tiny_reg"], str(L), str(cfg_path), str(NUM), str(out_path)], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-2000:]
+    reference_run("kgref_record", [tmp_models["tiny_reg"], L, cfg_path, NUM, out_path])
     want = _parse_text_dump(out_path.read_text())
     assert len(want) == 1
 

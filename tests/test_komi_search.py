@@ -90,9 +90,6 @@ def test_komi_searcher_schedules_jobs_over_its_slots():
         assert abs(v - (7.5 - (2.0 + i))) < 0.05, (i, v)
 
 
-REAL_NET_DRIVER = os.path.join(ROOT, "oracle", "_ref", "kgref_driver_b200")
-
-
 def _komitable_cases():
     import gzip, json
     return json.loads(gzip.open(os.path.join(ROOT, "tests", "golden", "komitable.json.gz"), "rb").read())["cases"]
@@ -156,20 +153,20 @@ def test_cpp_compute_lead_lands_on_the_reference_value_too(cpp_komi_driver):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not os.path.exists(REAL_NET_DRIVER), reason="oracle/_ref/kgref_driver_b200 not built (needs the reference sources at build time)")
 @pytest.mark.parametrize("stream,size,prefix_len,komi,visits", [("boardstream_9x9_multisuicide.npz", 9, 12, 7.5, 6), ("boardstream_9x9_multisuicide.npz", 9, 31, 0.5, 10),
                                                                ("boardstream_19x19_multisuicide.npz", 19, 40, 7.5, 6)])
 def test_lead_of_a_position_equals_the_reference_computeLead(golden_dir, stream, size, prefix_len, komi, visits):
     """PlayUtils::computeLead of the UNMODIFIED reference (its Search + NNEvaluator on libkgb200, fp32-equivalent, trained g170-b6c96 net,
-    symmetry 0, no cache) against the same computation as jobs on the device's side loop: the same komis are searched with the same few
-    visits, so the interpolated lead agrees to the evaluator's rounding."""
+    symmetry 0, no cache; its answers stored by tests/reference_runs.py) against the same computation as jobs on the device's side loop:
+    the same komis are searched with the same few visits, so the interpolated lead agrees to the evaluator's rounding."""
     sys.path.insert(0, golden_dir)
     import make_search_fixtures as F
     from katago_b200 import NeuralNet, SelfPlay
+    from reference_runs import reference_run
     model = os.path.join(golden_dir, "models", "g170-b6c96-s175395328-d26788732.bin.gz")
     moves = F.prefix_from_stream(stream, prefix_len)
     s = " ".join("pass" if m is None else f"{m[0]},{m[1]}" for m in moves)
-    out = subprocess.run([REAL_NET_DRIVER, "computelead", model, str(size), str(size), str(visits), repr(komi), s], capture_output=True, text=True, check=True).stdout
+    out = reference_run("kgref_driver_b200", ["computelead", model, size, size, visits, repr(komi), s])
     ref = float([ln.split()[1] for ln in out.splitlines() if ln.startswith("lead ")][0])
     lm = NeuralNet.loadModelFile(model)
     ctx = NeuralNet.createComputeContext([0], size, size, False, lm)

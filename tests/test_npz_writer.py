@@ -34,13 +34,13 @@ def test_written_file_has_the_reference_schema_and_round_trips(tmp_path):
     path = str(tmp_path / "rows.npz")
     assert W.write_npz(path, rows) == n
     with np.load(path) as z:
-        ref = np.load(os.path.join(os.environ.get("KATAGO_REF", "/root/reference"), "python/testdata/benchmark_data_1024.npz")) if os.path.exists(
-            "/root/reference/python/testdata/benchmark_data_1024.npz") else None
-        assert set(z.files) == set(W.schema())
+        # dtype and row shape of the reference's sample file python/testdata/benchmark_data_1024.npz (make_trainingdata_schema_fixture.py)
+        ref = json.load(open(os.path.join(GOLDEN, "trainingdata_schema.json")))
+        assert set(z.files) == set(W.schema()) == set(ref)
         for k, (descr, rest) in W.schema().items():
             assert z[k].dtype == np.dtype(descr) and z[k].shape == (n,) + tuple(rest)
-            if ref is not None and k != "globalTargetsNC":          # the sample file is format version 2 (64 global targets)
-                assert ref[k].dtype == z[k].dtype and ref[k].shape[1:] == z[k].shape[1:], k
+            if k != "globalTargetsNC":          # the sample file is format version 2 (64 global targets)
+                assert np.dtype(ref[k][0]) == z[k].dtype and tuple(ref[k][1]) == z[k].shape[1:], k
         # the reader's unpacking (python/katago/train/data_processing_pytorch.py:89-95) gives the planes back
         unpacked = np.unpackbits(z["binaryInputNCHWPacked"], axis=2)[:, :, :361]
         assert np.array_equal(unpacked, np.transpose(sp, (0, 2, 1)).astype(np.uint8))

@@ -438,9 +438,6 @@ def test_sgf_sink_appends_one_record_per_game(tmp_path):
     assert open(sink.path).read() == (d["sgf"] + "\n") * 2 and sink.count == 2
 
 
-DRIVER = os.path.join(ROOT, "oracle", "_ref", "kgref_driver")
-
-
 def _loader_case(which):
     """The .cfg variants both configuration loaders are compared on."""
     if which == "stock":
@@ -468,19 +465,19 @@ def _loader_case(which):
     return settings
 
 
-@pytest.mark.skipif(not os.path.exists(DRIVER), reason="oracle/_ref/kgref_driver not built")
 @pytest.mark.parametrize("which", ["stock", "every_key_changed", "almost_empty", "plain_fpu_weight", "dependent_defaults"])
 def test_config_mapping_agrees_with_the_reference_loader(tmp_path, which):
     """The same .cfg through the reference's own ConfigParser + Setup::loadSingleParams and integration/b200params.h
-    (`kgref_driver paramsmap`) and through selfplay_cli.py: every mapped field of kgb_selfplay_config agrees, defaults of
-    absent keys included, and the C++ side reports the same search options as not implemented."""
-    import json, subprocess
+    (`kgref_driver paramsmap`, answers stored by tests/reference_runs.py) and through selfplay_cli.py: every mapped field of
+    kgb_selfplay_config agrees, defaults of absent keys included, and the C++ side reports the same search options as not implemented."""
+    import json
     from katago_b200.nn_backend import SelfPlay
+    from reference_runs import reference_run
     settings = _loader_case(which)
     path = tmp_path / "c.cfg"
     path.write_text("".join(f"{k} = {v}\n" for k, v in settings.items()))
     kw, data, report = C.selfplay_kwargs_from_cfg(C.parse_cfg(str(path)))
-    ref = json.loads(subprocess.run([DRIVER, "paramsmap", str(path), str(kw["ko_rule"])], capture_output=True, text=True, check=True).stdout)
+    ref = json.loads(reference_run("kgref_driver", ["paramsmap", path, kw["ko_rule"]]))
     sig = inspect.signature(SelfPlay.__init__)
     eff = {k: v.default for k, v in sig.parameters.items() if v.default is not inspect._empty}
     eff.update(kw)
@@ -505,17 +502,17 @@ def cpp_host(tmp_path_factory):
     return str(exe)
 
 
-@pytest.mark.skipif(not os.path.exists(DRIVER), reason="oracle/_ref/kgref_driver not built")
 @pytest.mark.parametrize("which", ["stock", "every_key_changed", "almost_empty", "plain_fpu_weight", "dependent_defaults"])
 def test_cpp_host_config_mapping_agrees_with_the_reference_loader(tmp_path, cpp_host, which):
     """The C++ host reads a .cfg by the reference's key names itself (no reference headers): its kgb_selfplay_config agrees field by field
     with the reference's own loader mapped by integration/b200params.h, defaults of absent keys included."""
     import json, subprocess
+    from reference_runs import reference_run
     settings = {k: v.split(",")[0] for k, v in _loader_case(which).items() if k in C._SEARCH_KEYS or k in ("koRules", "multiStoneSuicideLegals", "numSearchThreads")}
     path = tmp_path / "c.cfg"
     path.write_text("".join(f"{k} = {v}\n" for k, v in settings.items()))
     mine = json.loads(subprocess.run([cpp_host, "-config", str(path), "-print-config"], capture_output=True, text=True, check=True).stdout)
-    ref = json.loads(subprocess.run([DRIVER, "paramsmap", str(path), str(mine["ko_rule"])], capture_output=True, text=True, check=True).stdout)
+    ref = json.loads(reference_run("kgref_driver", ["paramsmap", path, mine["ko_rule"]]))
     for k, v in ref.items():
         if k in ("unsupported", "komi", "multi_stone_suicide_legal"):      # rules are the game's, not the search parameters'
             continue
